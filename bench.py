@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - end-to-end FPS of the SMAP inference hot path (backbone + association + 3D lift) on B200.
 
-Contract (driver): `python bench.py --gpus N --steps K --warmup W [--impl reference]`, under torchrun for
+Usage: `python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]`, under torchrun for
 N > 1; one JSON line on stdout from rank 0.
 
 A "step" = one pass of the whole hot path over one batch of B synthetic 832x512 frames per GPU
@@ -16,6 +16,10 @@ B frames and the per-image skeleton records are exchanged with ONE NCCL all-gath
           MEASURED_PEAKS.json bf16_tflops_sustained.
           In bf16x3 mode every algorithmic FLOP is issued as 3 tensor-core FLOPs, so the tensor pipe runs at
           3 x frac of the bf16 peak.
+  --dump-outputs DIR : after the timed steps, rank 0 writes what the last timed device-resident step returned (the
+          skeleton records of its B frames, all ranks' with N > 1) as DIR/pred2d.npy (float32 [F,127,15,4]), pred3d.npy
+          (float64 [F,127,15,4]), root_depth.npy (float64 [F,127]) and count.npy (float64 [F]).  Inputs and weights are
+          seeded, so the same arguments give the same inputs on every run and two builds can be compared array by array.
   cpu_baseline : the CPU oracle of the same path (oracle/: PyTorch fp32 backbone on all cores + C++ association
           + numpy lift) on a bounded sample of the same workload.
 `--impl reference` times that CPU oracle alone (the reference has no GPU-free path of its own for the association
@@ -54,7 +58,23 @@ def parse():
     ap.add_argument("--profile-csv", default="")
     ap.add_argument("--ncu-one-step", action="store_true",
                     help="bracket exactly one device-resident step with cudaProfilerStart/Stop and exit (for ncu --profile-from-start off)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the records of the last timed step as DIR/<field>.npy (float32/float64)")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "smap_b200":
+        ap.error("--dump-outputs needs --impl smap_b200")
+    return args
+
+
+def dump_outputs(out_dir, rec):
+    """Records (uint8 [F, RECORD_BYTES], any device) -> out_dir/{pred2d,pred3d,root_depth,count}.npy."""
+    from smap_b200.engine import records_to_numpy
+
+    os.makedirs(out_dir, exist_ok=True)
+    r = records_to_numpy(rec)
+    for name in ("pred2d", "pred3d", "root_depth"):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(r[name]))
+    np.save(os.path.join(out_dir, "count.npy"), r["count"].astype(np.float64))
 
 
 def measured_peaks():
@@ -412,6 +432,8 @@ def run_ours(args):
     ms_dev, wall_dev = timed(run_device, args.steps)
     per_rank_ms = timed.per_rank
     launches = sum(e.launch_count() for e in engines) - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dev_outs[(args.steps - 1) % NE])  # step i wrote dev_outs[i % NE]
 
     run_host(max(DEPTH, args.warmup))  # slot buffers + graphs for the slot pointers, then the host warm-up
     torch.cuda.synchronize()

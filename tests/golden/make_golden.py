@@ -10,6 +10,7 @@ build container.  The fixtures travel to the GPU box; /root/reference does not.
                        exps/stage3_root2/test.py:116-134 does, including cv2 INTER_NEAREST up-sampling.
 
   lift_gt_cases.npz  : the same with ground truth (register_pred's matching branch, test_util.py:21-39, float64 rows).
+  shim_schema.npz    : the state-dict schema and seeded random initialisation of the reference SMAP and RefineNet.
 
 Run:  python tests/golden/make_golden.py
 """
@@ -174,12 +175,17 @@ def golden_lift_gt():
 
 def golden_refine():
     """refine_cases.npz: outputs of the unmodified model/refinenet.py + test_util.lift_and_refine_3d_pose on the lift
-    goldens (the 2D/3D poses the reference lift produced), with seeded weights."""
+    goldens (the 2D/3D poses the reference lift produced), with seeded weights.  torch.nn.functional.linear is replaced
+    by oracle.refine_torch.linear (the same float32 linear with one fixed summation order), so that the fixture does not
+    depend on which CPU and BLAS kernel made it."""
     _reference_env()
     import test_util as T
     from model.refinenet import RefineNet
 
     from cases import N_LIFT_CASES, refine_state_dict
+    from oracle.refine_torch import linear
+
+    torch.nn.functional.linear = linear
 
     lift = np.load(os.path.join(HERE, "lift_cases.npz"))
     net = RefineNet().eval()
@@ -251,8 +257,34 @@ def golden_preprocess():
     print("preprocess golden:", len(out), "cases")
 
 
+def golden_schema():
+    """shim_schema.npz: keys, shapes, dtypes and SHA-256 (first 16 hex digits) of the values of the state dicts of the
+    unmodified model/smap.py SMAP (torch.manual_seed(0)) and model/refinenet.py RefineNet (torch.manual_seed(3)) right
+    after construction, i.e. their random initialisation."""
+    import hashlib
+
+    from model.refinenet import RefineNet
+    from model.smap import SMAP
+
+    cfg = NS(MODEL=NS(STAGE_NUM=3, UPSAMPLE_CHANNEL_NUM=256), DATASET=NS(KEYPOINT=NS(NUM=15), PAF=NS(NUM=14)),
+             OUTPUT_SHAPE=(128, 208), LOSS=NS(OHKM=True, TOPK=8, COARSE_TO_FINE=True))
+    out = {}
+    for name, make, seed in (("smap", lambda: SMAP(cfg), 0), ("refinenet", RefineNet, 3)):
+        torch.manual_seed(seed)
+        sd = make().state_dict()
+        out[name + "_keys"] = np.array(list(sd.keys()))
+        out[name + "_shapes"] = np.array(["x".join(map(str, v.shape)) for v in sd.values()])
+        out[name + "_dtypes"] = np.array([str(v.dtype) for v in sd.values()])
+        out[name + "_sha256"] = np.array([hashlib.sha256(v.contiguous().numpy().tobytes()).hexdigest()[:16]
+                                          for v in sd.values()])
+    np.savez_compressed(os.path.join(HERE, "shim_schema.npz"), **out)
+    print("schema golden:", len(out["smap_keys"]), "SMAP tensors,", len(out["refinenet_keys"]), "RefineNet tensors")
+
+
 if __name__ == "__main__":
-    which = sys.argv[1:] or ["backbone", "lift", "lift_gt", "refine", "json", "preprocess"]
+    which = sys.argv[1:] or ["backbone", "lift", "lift_gt", "refine", "json", "preprocess", "schema"]
+    if "schema" in which:
+        golden_schema()
     if "lift_gt" in which:
         golden_lift_gt()
     if "preprocess" in which:

@@ -1,10 +1,13 @@
-"""GPU: association kernels (through the C ABI) bit-exact against the CPU oracle and - when
-oracle/_ref/dapalib_ref*.so is present - against the UNMODIFIED reference extension running on this GPU."""
+"""GPU: association kernels (through the C ABI) bit-exact against the CPU oracle and against the outputs of the
+UNMODIFIED reference extension on a B200 (tests/golden/assoc_ref_cases.npz, tests/golden/make_golden_assoc.py)."""
+import hashlib
+import os
+
 import numpy as np
 import pytest
 import torch
 
-from oracle import assoc, build_ref
+from oracle import assoc
 from smap_b200.synth import make_scene
 
 pytestmark = pytest.mark.gpu
@@ -21,8 +24,8 @@ def eng():
 
 
 @pytest.fixture(scope="module")
-def ref_mod():
-    return build_ref.load_ref()
+def ref_gold():
+    return np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "assoc_ref_cases.npz"))
 
 
 def scenes(seeds, persons=15):
@@ -135,47 +138,59 @@ def test_batch_invariance(eng):
         assert torch.equal(b1[0], b8[i]) and c1[0] == c8[i]
 
 
-# ---------------- the real reference on this GPU ----------------
-def test_against_unmodified_reference_extension(eng, ref_mod):
-    if ref_mod is None:
-        pytest.skip("oracle/_ref/dapalib_ref*.so not built (needs /root/reference at build time)")
+# ---------------- the unmodified reference extension (its outputs on a B200, stored) ----------------
+def reference_cases():
     sets = [scenes(range(40, 44))[:2], random_heatmaps(5, B=2)]
     ec = edge_cases()
     for name in ("plateau_border_threshold", "saturated_127_peaks", "coincident_and_near", "empty"):
         sets.append((ec[name][None], np.random.default_rng(3).uniform(0.5, 3, (1, H, W)).astype(np.float32)))
-    for hms, rd in sets:
+    return sets
+
+
+def oracle_cases():
+    return scenes(range(50, 53))[:2]
+
+
+def _sha(*arrays):
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def test_against_unmodified_reference_extension(eng, ref_gold):
+    pairs = [0, 1, 0, 2, 0, 9, 9, 10, 10, 11, 0, 3, 3, 4, 4, 5, 2, 12, 12, 13, 13, 14, 2, 6, 6, 7, 7, 8]
+    for c, (hms, rd) in enumerate(reference_cases()):
         th = torch.from_numpy(hms).cuda()
         bodies, counts = eng.connect(th, torch.from_numpy(rd).cuda())
         peaks, scores = eng.extract(th)
         torch.cuda.synchronize()
         for b in range(hms.shape[0]):
-            pc, sc = ref_mod.extract(th[b].contiguous())
+            key = "c%d_b%d_" % (c, b)
+            assert _sha(hms[b], rd[b]) == str(ref_gold[key + "input_sha256"]), "input generators changed (case %d)" % c
+            npk = ref_gold[key + "npeaks"]
+            ref_peaks = np.split(ref_gold[key + "peaks"], np.cumsum(npk)[:-1])
             for j in range(15):
                 n = int(peaks[b, j, 0, 0].item())
-                assert pc[j].shape[0] == n
-                assert torch.equal(pc[j], peaks[b, j, 1:n + 1].cpu())
-            pairs = [0, 1, 0, 2, 0, 9, 9, 10, 10, 11, 0, 3, 3, 4, 4, 5, 2, 12, 12, 13, 13, 14, 2, 6, 6, 7, 7, 8]
+                assert npk[j] == n
+                assert np.array_equal(ref_peaks[j], peaks[b, j, 1:n + 1].cpu().numpy())
             for l in range(14):
-                nA, nB = pc[pairs[2 * l]].shape[0], pc[pairs[2 * l + 1]].shape[0]
-                assert torch.equal(sc[l], scores[b, l, :nA, :nB].cpu()), "pair scores differ from the reference"
-            ref_b = ref_mod.connect(th[b].contiguous(), torch.from_numpy(rd[b]), 2, True)
+                nA, nB = int(npk[pairs[2 * l]]), int(npk[pairs[2 * l + 1]])
+                assert _sha(scores[b, l, :nA, :nB].cpu().numpy()) == ref_gold[key + "scores_sha256"][l], \
+                    "pair scores differ from the reference"
+            ref_b = ref_gold[key + "bodies"]
             n = int(counts[b].item())
-            if n == 0:
-                assert ref_b.numel() == 0
-            else:
-                assert tuple(ref_b.shape) == (n, 15, 4)
-                assert torch.equal(ref_b, bodies[b, :n].cpu()), "bodies differ from the reference"
+            assert ref_b.shape == (n, 15, 4)
+            assert np.array_equal(ref_b, bodies[b, :n].cpu().numpy()), "bodies differ from the reference"
 
 
-def test_oracle_matches_unmodified_reference_extension(ref_mod):
+def test_oracle_matches_unmodified_reference_extension(ref_gold):
     """Pins the CPU oracle itself against the reference (SURVEY.md 8(c))."""
-    if ref_mod is None:
-        pytest.skip("oracle/_ref/dapalib_ref*.so not built")
-    hms, rd, _ = scenes(range(50, 53))
+    hms, rd = oracle_cases()
     for b in range(3):
-        ref_b = ref_mod.connect(torch.from_numpy(hms[b]).cuda(), torch.from_numpy(rd[b]), 2, True)
+        assert _sha(hms[b], rd[b]) == str(ref_gold["o_b%d_input_sha256" % b]), "input generators changed"
         ob = assoc.connect(hms[b], rd[b])
-        assert np.array_equal(ref_b.numpy(), ob)
+        assert np.array_equal(ref_gold["o_b%d_bodies" % b], ob)
 
 
 # ---------------- lift ----------------

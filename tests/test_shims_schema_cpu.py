@@ -1,13 +1,15 @@
 """CPU: the drop-in modules expose exactly the reference's state-dict schema (keys, order, shapes) and random init.
 
-When /root/reference is mounted (the build container) the comparison is made against the reference modules themselves;
-everywhere else against the key lists the oracle restates (oracle/smap_torch.py, oracle/refine_torch.py), which
-tests/test_oracle_golden.py pins to the reference.  No forward pass: the shims need a B200 for that."""
+Compared against the key lists the oracle restates (oracle/smap_torch.py, oracle/refine_torch.py), which
+tests/test_oracle_golden.py pins to the reference, and against tests/golden/shim_schema.npz: the keys, shapes, dtypes and
+value digests of the reference modules' own state dicts (tests/golden/make_golden.py).  No forward pass: the shims need
+a B200 for that."""
+import hashlib
 import os
 import sys
 import types
 
-import pytest
+import numpy as np
 import torch
 
 from oracle import refine_torch
@@ -15,7 +17,6 @@ from smap_b200 import schema
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SHIMS = os.path.join(ROOT, "smap_b200", "shims")
-REF = "/root/reference"
 
 
 def _cfg():
@@ -51,28 +52,25 @@ def test_shim_schemas_match_the_restated_key_lists():
     assert [(k, tuple(v.shape)) for k, v in r.state_dict().items()] == [(k, tuple(s)) for k, s in refine_torch.refine_keys()]
 
 
-@pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "model")), reason="reference not mounted")
+def _check_against_golden(gold, name, sd):
+    keys = list(sd.keys())
+    assert keys == list(gold[name + "_keys"])
+    for k, shape, dtype, digest in zip(keys, gold[name + "_shapes"], gold[name + "_dtypes"], gold[name + "_sha256"]):
+        v = sd[k]
+        assert "x".join(map(str, v.shape)) == shape and str(v.dtype) == dtype, k
+        assert hashlib.sha256(v.contiguous().numpy().tobytes()).hexdigest()[:16] == digest, "random init differs at " + k
+
+
 def test_shims_match_the_reference_modules_key_for_key_and_init_for_init():
-    ref_smap, ref_refine = _import_from(REF, ["model.smap", "model.refinenet"])
+    gold = np.load(os.path.join(ROOT, "tests", "golden", "shim_schema.npz"))
     shim_smap, shim_refine = _import_from(SHIMS, ["model.smap", "model.refinenet"])
-    torch.manual_seed(0)
-    a = ref_smap.SMAP(_cfg()).state_dict()
-    torch.manual_seed(0)
-    b = shim_smap.SMAP(_cfg()).state_dict()
-    assert list(a.keys()) == list(b.keys())
-    for k in a:
-        assert a[k].shape == b[k].shape and a[k].dtype == b[k].dtype, k
-        assert torch.equal(a[k], b[k]), "random init differs at " + k   # same construction order -> same RNG stream
+    torch.manual_seed(0)  # same construction order as the reference -> same RNG stream
+    _check_against_golden(gold, "smap", shim_smap.SMAP(_cfg()).state_dict())
     torch.manual_seed(3)
-    ra = ref_refine.RefineNet().state_dict()
-    torch.manual_seed(3)
-    rb = shim_refine.RefineNet().state_dict()
-    assert list(ra.keys()) == list(rb.keys())
-    for k in ra:
-        assert ra[k].shape == rb[k].shape and torch.equal(ra[k], rb[k]), k
-    # strict loading in both directions
-    shim_refine.RefineNet().load_state_dict(ra)
-    ref_refine.RefineNet().load_state_dict(rb)
+    _check_against_golden(gold, "refinenet", shim_refine.RefineNet().state_dict())
+    # strict loading of a state dict with the reference's keys and shapes
+    ref_sd = {k: torch.zeros([int(d) for d in s.split("x") if d]) for k, s in zip(gold["refinenet_keys"], gold["refinenet_shapes"])}
+    shim_refine.RefineNet().load_state_dict(ref_sd)
 
 
 def test_oracle_and_product_generators_agree_bit_for_bit():
